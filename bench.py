@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the two hot paths (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of FeatureTracker::trackImage over one batch of FRAMES_PER_STEP = 100 consecutive 640x480 RGB-D frames
 of a synthetic stream with 150 features (BASELINE.json configs[1], "C2"), submitted as ONE library call
@@ -22,6 +22,10 @@ reported.
 
 --impl reference times the reference's CPU path: the reference cannot be compiled here (ROS / Eigen / Ceres / OpenCV C++
 absent), so this is the restatement on the same three OpenCV entry points (kind "port"), all host threads.
+
+--dump-outputs DIR writes, as float64 .npy files, what the last timed step of the headline (device-resident) run returned to
+its caller: the observations, inlier masks and counters of its FRAMES_PER_STEP frames (rank 0's stream).  The inputs depend
+only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -195,17 +199,21 @@ class Stream:
         p8 = idc_params8()
         p8 = [p8[0] * sc, p8[1] * sc, p8[2] * sc, p8[3] * sc] + p8[4:]
         self.tr = FeatureTracker(wl["w"], wl["h"], p8, wl["max_cnt"], wl["min_dist"], 1, 1, device=device)
-        self.ring, self.k, self.dev_ms = ring, offset, 0.0
+        self.ring, self.k, self.dev_ms, self.last_out = ring, offset, 0.0, None
 
-    def run(self, n_steps, mode):
-        """n_steps batches of FRAMES_PER_STEP frames; returns the device time of the run (CUDA events on the tracker's streams)."""
+    def run(self, n_steps, mode, keep_last=False):
+        """n_steps batches of FRAMES_PER_STEP frames; returns the device time of the run (CUDA events on the tracker's streams).
+        keep_last: the last batch also copies its results out to the caller (self.last_out, as trackBatch returns them)."""
         g, d = self.ring.ptr[mode]
         n = self.ring.n
         self.tr.timer_start()
-        for _ in range(n_steps):
+        for s in range(n_steps):
             idx = [tri(self.k + j, n) for j in range(FRAMES_PER_STEP)]
             times = [(self.k + j) / 30.0 for j in range(FRAMES_PER_STEP)]
-            self.tr.trackBatch(times, [g[i] for i in idx], [d[i] for i in idx], on_device=(mode == "device"), want=False)
+            want = keep_last and s == n_steps - 1
+            out = self.tr.trackBatch(times, [g[i] for i in idx], [d[i] for i in idx], on_device=(mode == "device"), want=want)
+            if want:
+                self.last_out = out
             self.k += FRAMES_PER_STEP
         self.dev_ms = self.tr.timer_stop()
         return self.dev_ms
@@ -229,15 +237,16 @@ def run_multi(streams, n_steps, mode):
         s.dev_ms = s.tr.timer_stop()
 
 
-def timed(streams, n_steps, mode, barrier, sampler=None, threads=False):
+def timed(streams, n_steps, mode, barrier, sampler=None, threads=False, keep_last=False):
     """K steps on every stream of this rank; wall clock between barriers.  Several streams: one host thread and
     gf_tracker_track_batch_multi, or (threads=True, for comparison) one host thread per stream."""
+    assert not keep_last or len(streams) == 1
     barrier()
     if sampler is not None:
         sampler.active = True
     t0 = time.perf_counter()
     if len(streams) == 1:
-        streams[0].run(n_steps, mode)
+        streams[0].run(n_steps, mode, keep_last)
     elif not threads:
         run_multi(streams, n_steps, mode)
     else:
@@ -253,12 +262,13 @@ def timed(streams, n_steps, mode, barrier, sampler=None, threads=False):
     return el, max(s.dev_ms for s in streams)
 
 
-def fe_line(wl, rings, device, n_streams, steps, warmup, barrier, sampler, reduce_max, threads=False):
+def fe_line(wl, rings, device, n_streams, steps, warmup, barrier, sampler, reduce_max, threads=False, keep_last=False):
+    """keep_last: "last_step" of the result is what the last device-resident timed step returned (see Stream.run)."""
     streams = [Stream(rings[0], wl, device, offset=17 * s) for s in range(n_streams)]
     from ground_fusion_b200 import _lib
     timed(streams, warmup, "device", barrier, threads=threads)
     l0 = _lib.lib().gf_kernel_launch_count()
-    el_dev, ms_dev = timed(streams, steps, "device", barrier, sampler, threads=threads)
+    el_dev, ms_dev = timed(streams, steps, "device", barrier, sampler, threads=threads, keep_last=keep_last)
     launches = _lib.lib().gf_kernel_launch_count() - l0
     timed(streams, max(1, warmup // 2), "host", barrier, threads=threads)
     el_e2e, ms_e2e = timed(streams, steps, "host", barrier, sampler, threads=threads)
@@ -269,7 +279,30 @@ def fe_line(wl, rings, device, n_streams, steps, warmup, barrier, sampler, reduc
     frames = n_streams * steps * FRAMES_PER_STEP
     return {"value": frames / el_dev, "e2e": frames / el_e2e, "ms_per_step": 1e3 * el_dev / steps, "ms_per_step_e2e": 1e3 * el_e2e / steps,
             "device_ms_per_step": ms_dev / steps, "device_ms_per_step_e2e": ms_e2e / steps, "streams_per_gpu": n_streams, "gpu_launches": int(launches),
-            "mean_features_tracked": float(np.mean([i["n_tracked"] for i in infos])), "mean_lk_iterations": float(np.mean([i["lk_iterations"] for i in infos]))}
+            "mean_features_tracked": float(np.mean([i["n_tracked"] for i in infos])), "mean_lk_iterations": float(np.mean([i["lk_iterations"] for i in infos])),
+            "last_step": streams[0].last_out}
+
+
+def dump_outputs(path, batch, max_cnt):
+    """One trackBatch result (per frame: observations, inlier mask, counters) as float64 arrays padded to max_cnt per frame:
+    n_obs[f], obs_id[f, i] (-1 past n_obs), obs_track_cnt[f, i], obs_v[f, i, 8] (gf_obs.v: x_n y_n 1 u v vx_n vy_n depth_m),
+    n_prev[f], status[f, i] (0 past n_prev), info[f, :] (gf_track_info in declaration order)."""
+    from ground_fusion_b200._lib import TrackInfo
+    fields = [name for name, _ in TrackInfo._fields_]
+    n = len(batch)
+    a = {"n_obs": np.zeros(n), "obs_id": np.full((n, max_cnt), -1.0), "obs_track_cnt": np.zeros((n, max_cnt)),
+         "obs_v": np.zeros((n, max_cnt, 8)), "n_prev": np.zeros(n), "status": np.zeros((n, max_cnt)), "info": np.zeros((n, len(fields)))}
+    for f, (obs, status, info) in enumerate(batch):
+        m, p = len(obs), len(status)
+        a["n_obs"][f], a["n_prev"][f] = m, p
+        a["obs_id"][f, :m] = obs["id"]
+        a["obs_track_cnt"][f, :m] = obs["track_cnt"]
+        a["obs_v"][f, :m] = obs["v"]
+        a["status"][f, :p] = status
+        a["info"][f] = [info[k] for k in fields]
+    os.makedirs(path, exist_ok=True)
+    for name, arr in a.items():
+        np.save(os.path.join(path, name + ".npy"), arr)
 
 
 def ba_bench(device, clocks_mhz, n_windows=8, reps=200, cpu_seconds=8.0):
@@ -414,7 +447,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cpu-seconds", type=float, default=8.0)
     ap.add_argument("--no-extras", action="store_true", help="only the headline C2 line (no stream sweep, C3/C4, BA)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the headline run returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and at least one timed step")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     wl = WORKLOADS["C2"]
     cfg = {"workload": wl["name"], "frames_per_step": FRAMES_PER_STEP, "frames_ring": wl["ring"],
@@ -473,8 +509,10 @@ def main():
     if rank == 0:
         sampler = ClockSampler(local); sampler.start()
     ring = Ring(rank, wl, torch)
-    head = fe_line(wl, [ring], local, 1, args.steps, args.warmup, barrier, sampler, reduce_max)
+    head = fe_line(wl, [ring], local, 1, args.steps, args.warmup, barrier, sampler, reduce_max, keep_last=bool(args.dump_outputs))
     clocks = sampler.summary() if sampler is not None else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, head["last_step"], wl["max_cnt"])
 
     extra = {}
     if world > 1 and not args.no_extras:
